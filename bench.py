@@ -7,11 +7,13 @@ synthetic VOC-shaped images (BASELINE.json configs[1]) -- backbone + heads
 batch-parallel, one NCCL all-gather of the detection records per step).
 
   python bench.py --gpus N --steps K --warmup W          # this framework
+  python bench.py ... --dump-outputs DIR                 # + the last timed step's detections as DIR/*.npy
   python bench.py --impl reference --gpus N ...          # the reference's CPU path
                                                          # (oracle port: TF1.13 cannot run here)
 One JSON line on stdout (rank 0).
 """
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -83,6 +85,7 @@ class ClockSampler:
                 ["nvidia-smi", "-i", str(self.index), "--query-gpu=" + self.Q,
                  "--format=csv,noheader,nounits", "-lms", "100"],
                 stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self._kill)  # an exception inside a timed leg must not leave nvidia-smi running
             self.t = threading.Thread(target=self._read, daemon=True)
             self.t.start()
         except Exception:
@@ -91,6 +94,11 @@ class ClockSampler:
     def _read(self):
         for line in self.proc.stdout:
             self.lines.append(line.strip())
+
+    def _kill(self):
+        if self.proc.poll() is None:
+            self.proc.kill()
+            self.proc.wait()
 
     def stop(self):
         if self.proc is None:
@@ -263,6 +271,20 @@ def timed_ops(net, pick, reps=5):
             med([a.elapsed_time(b) for a, b in dec]), med([a.elapsed_time(b) for a, b in nms]))
 
 
+def dump_detections(out_dir, name, tail):
+    """What a caller of the timed step receives: the Detections of the step's packed records (scores [B,D],
+    boxes [B,D,4] as y1,x1,y2,x2, class ids [B,D], counts [B]), slots past each image's count zeroed, written as
+    float32 to out_dir/<name>_<array>.npy.  Inputs and weights are seeded, so two builds can be compared file by file."""
+    from odt_b200.engine import unpack_records
+    det = unpack_records(tail.rec.cpu().numpy(), tail.p.cap)
+    valid = np.arange(det.scores.shape[1])[None, :] < det.count[:, None]
+    arrays = {"scores": np.where(valid, det.scores, 0), "boxes": np.where(valid[..., None], det.boxes, 0),
+              "class_id": np.where(valid, det.class_id, 0), "count": det.count}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, "%s_%s.npy" % (name, k)), np.asarray(v, np.float32))
+
+
 def tail_launch_floor_us():
     """The same two tail launches (memset + decode, memsets + NMS) on a 32-row input: the launch-bound floor."""
     import numpy as np
@@ -331,6 +353,8 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-retinanet", action="store_true", help="skip the second workload (RetinaNet-800 B=16)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the detections of each workload's last timed step to DIR/*.npy")
     args = ap.parse_args()
     assert args.warmup >= 0 and args.steps >= 1
 
@@ -380,16 +404,18 @@ def main():
     def time_resident(net, gathered, sampler=None):
         """W warm-up + K timed device-resident steps (graph replay + the records' all-gather at N > 1).  Default: the
         two-stage pipeline of the engine (decode + NMS + gather of step i on a second stream under the first
-        convolutions of step i+1, everything the tail touches double-buffered); ODT_PIPELINE=0: one graph per step."""
+        convolutions of step i+1, everything the tail touches double-buffered); ODT_PIPELINE=0: one graph per step.
+        Returns (ms of the K steps, the Tail holding the last step's records)."""
         pipelined = os.environ.get("ODT_PIPELINE", "1") != "0"
         if pipelined:
             net.capture_pipelined()
         counter = [0]
+        last = [net.tail]
 
         def step():
             if pipelined:
-                net.run_pipelined(counter[0] & 1,
-                                  (lambda t: od.gather_records(t.rec, out=gathered)) if world > 1 else None)
+                last[0] = net.run_pipelined(counter[0] & 1,
+                                            (lambda t: od.gather_records(t.rec, out=gathered)) if world > 1 else None)
                 counter[0] += 1
                 return
             net.run()
@@ -417,7 +443,7 @@ def main():
             net.join_pipelined()  # the closing event waits for the last tails as well
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1))
+        return max_over_ranks(e0.elapsed_time(e1)), last[0]
 
     def time_e2e(model, images, sampler=None):
         """Public API, host buffers: pinned H2D of every step's images + D2H of every step's records inside
@@ -463,8 +489,10 @@ def main():
     torch.cuda.synchronize()
     sampler = ClockSampler(local)
     sampler.start()  # started before the warm-up so that samples exist for short timed regions
-    ms_total = time_resident(net, gathered, sampler)
+    ms_total, last_tail = time_resident(net, gathered, sampler)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_detections(args.dump_outputs, "ssd300", last_tail)
     ms_step = ms_total / K
     value = world * BATCH * K / (ms_total / 1e3)
     from odt_b200.engine import ConvOp
@@ -526,15 +554,18 @@ def main():
             tdist.broadcast(tt, 0)
             thr = float(tt.item()) if tt.item() >= 0 else None
         if thr is not None:
-            rnet.tail.p.score_thr = thr
+            # the Tail's own attribute too: capture_pipelined() prepares the second pipeline slot's tail from it
+            rnet.tail.score_thr = rnet.tail.p.score_thr = thr
             rmodel.nms_score_threshold = thr
         rnet.capture()
         rg = (torch.empty((world * RETINA_BATCH, rnet.tail.rec.shape[1]), dtype=torch.float32, device="cuda")
               if world > 1 else None)
         rs1 = ClockSampler(local)
         rs1.start()
-        r_ms_total = time_resident(rnet, rg, rs1)
+        r_ms_total, r_last_tail = time_resident(rnet, rg, rs1)
         r_clocks = rs1.stop()
+        if args.dump_outputs and rank == 0:
+            dump_detections(args.dump_outputs, "retinanet800", r_last_tail)
         r_ms_step = r_ms_total / K
         r_tc_ms, r_dec_ms, r_nms_ms = timed_ops(rnet, is_tc)
         rs2 = ClockSampler(local)
